@@ -70,6 +70,10 @@ def parse_args():
     ap.add_argument("--lmm-markers", type=int, default=0,
                     help="also run the GRM-covariance LMM engine (eigen-rotation GEMM + per-marker delta search) "
                          "on this many markers")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the per-marker outputs of the last timed step as DIR/<name>.npy "
+                         "(float64, markers with a result only, their 0-based indices in DIR/marker_index.npy; at most "
+                         "64 MB in all, a fixed seeded sample of the markers beyond that)")
     return ap.parse_args()
 
 
@@ -158,6 +162,41 @@ def log(msg: str):
 
 def shard_bounds(p: int, world: int, rank: int):
     return (p * rank) // world, (p * (rank + 1)) // world
+
+
+DUMP_BYTES = 64_000_000  # --dump-outputs: all files together, .npy headers included
+
+
+def dump_outputs(out_dir: str, arrays: dict, p: int, j0: int, world: int):
+    """Writes per-marker arrays (this rank holds markers j0 .. j0 + len - 1 of p) as out_dir/<name>.npy in float64 and
+    global marker order, from rank 0 of the `world` ranks, with the 0-based indices of the markers written as
+    marker_index.npy.  Only markers with a result are written: the scan leaves NaN at markers removed by the
+    fixed-locus filter and at degenerate ones, and a caller's fit holds no entry for them.  When the arrays of all p
+    markers would exceed DUMP_BYTES, a fixed seeded sample of the markers is taken (the same one in every array)."""
+    k = len(arrays) + 1  # + marker_index
+    if 8 * k * p + 1024 * k <= DUMP_BYTES:
+        idx = np.arange(p)
+    else:
+        m = (DUMP_BYTES - 1024 * k) // (8 * k)
+        idx = np.sort(np.random.default_rng(SEED).choice(p, m, replace=False))
+    p_loc = len(next(iter(arrays.values())))
+    mine = idx[(idx >= j0) & (idx < j0 + p_loc)]
+    local = {name: np.asarray(a, dtype=np.float64)[mine - j0] for name, a in arrays.items()}
+    local["marker_index"] = mine.astype(np.float64)
+    if world > 1:  # contiguous column blocks: rank order is marker order
+        import torch.distributed as dist
+
+        parts = [None] * world
+        dist.all_gather_object(parts, local)
+        local = {name: np.concatenate([q[name] for q in parts]) for name in local}
+    if int(os.environ.get("RANK", "0")) != 0:
+        return
+    has_result = np.logical_and.reduce([np.isfinite(local[name]) for name in arrays])
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in local.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a[has_result])
+    log(f"outputs of the last timed step: {int(has_result.sum())} markers with a result of {local['marker_index'].size} "
+        f"{'' if idx.size == p else 'sampled '}of {p} -> {out_dir}")
 
 
 # --------------------------------------------------------------------------------------
@@ -253,8 +292,10 @@ def run_reference(args):
         cbind.gwasols_raw(A[:, : min(markers, 2048)], ys, pc)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        cbind.gwasols_raw(A, ys, pc)
+        stat_ols, stat_lmm, _ = cbind.gwasols_raw(A, ys, pc)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"stat_ols": stat_ols, "stat_lmm": stat_lmm}, markers, 0, 1)
     value = markers * args.steps / dt
     sample = f"{markers} of {args.p} markers per step (n={n}), C/OpenMP restatement of gwas.jl:112-115,:129,:241-245"
     line = {
@@ -355,6 +396,10 @@ def main():
     dev_s, wall, main_avg_ms = (float(x) for x in t.cpu())
     value = p * args.steps / dev_s
     wall_value = p * args.steps / wall
+    if args.dump_outputs:  # before the packed-copy section below reuses the output buffers
+        dump_outputs(args.dump_outputs, {"beta": outs["beta"].cpu(), "se": outs["se"].cpu(), "stat": outs["stat"].cpu(),
+                                         "neglog10p": outs["nlp"].cpu(), "mean": outs["mean"].cpu(),
+                                         "sd": outs["sd"].cpu()}, p, j0, world)
 
     peak, peak_src = measured_peaks()
     algo_bytes = 8.0 * n * p_loc  # SURVEY 8d: 8n bytes per marker, each genotype read once
