@@ -2014,53 +2014,48 @@ int gbm_scan_host(const double* A, int64_t n, int64_t p, int64_t lda, const doub
 // ------------------------------------------------------------------------------------
 // GRM-covariance LMM scan (rotation + per-marker delta search)
 // ------------------------------------------------------------------------------------
-struct gbm_lmm_plan {
-  int64_t n = 0, ldu = 0;
-  int Q0 = 1;
-  double* dU = nullptr;   // eigenvectors, n x n (ldu)
-  double* dS = nullptr;   // eigenvalues ascending
-  double* dYr = nullptr;  // U'y
-  double* dCr = nullptr;  // U'[1, C], n x Q0 (ld n)
-  double lam0 = 0.0;
-  double s_min = 0.0;     // smallest eigenvalue (negative for an indefinite K)
-};
+namespace gbm {
 
-extern "C" {
-
-int gbm_lmm_plan_create(const double* K, int64_t n, const double* y, const double* C, int64_t k, int64_t ldc,
-                        gbm_lmm_plan** plan_out, double* eig_ms, double* null_log_delta) {
-  GBM_API_BEGIN
-  require_ready();
-  if (!K || !y || !plan_out || n < 4) GBM_THROW(GBM_ERR_ARGUMENT, "gbm_lmm_plan_create: bad arguments");
-  if (k < 0 || k > 2 || (k > 0 && (!C || ldc < n)))
-    GBM_THROW(GBM_ERR_ARGUMENT, "gbm_lmm_plan_create: 0..2 covariates besides the intercept are supported");
-  if (n > 2147483647) GBM_THROW(GBM_ERR_ARGUMENT, "n too large for cuSOLVER");
-  State& st = state();
-  reset_timing();
+gbm_lmm_plan* lmm_plan_alloc(int64_t n, int Q0) {
   std::unique_ptr<gbm_lmm_plan> pl(new gbm_lmm_plan);
   pl->n = n;
   pl->ldu = round_up(n, 16);
-  pl->Q0 = static_cast<int>(k) + 1;
-  const int Q0 = pl->Q0;
+  pl->Q0 = Q0;
   auto dalloc = [&](double** p, size_t count) {
     cudaError_t e = cudaMalloc(reinterpret_cast<void**>(p), sizeof(double) * count);
-    if (e != cudaSuccess) GBM_THROW(GBM_ERR_CUDA, std::string("cudaMalloc failed: ") + cudaGetErrorString(e));
-  };
-  struct Guard {
-    gbm_lmm_plan* p;
-    ~Guard() {
-      if (p) {
-        cudaFree(p->dU); cudaFree(p->dS); cudaFree(p->dYr); cudaFree(p->dCr);
-      }
+    if (e != cudaSuccess) {
+      lmm_plan_destroy(pl.release());
+      GBM_THROW(GBM_ERR_CUDA, std::string("cudaMalloc failed: ") + cudaGetErrorString(e));
     }
-  } guard{pl.get()};
+  };
   dalloc(&pl->dU, static_cast<size_t>(pl->ldu) * n);
   dalloc(&pl->dS, n);
   dalloc(&pl->dYr, n);
   dalloc(&pl->dCr, static_cast<size_t>(n) * Q0);
+  return pl.release();
+}
+
+void lmm_plan_destroy(gbm_lmm_plan* pl) {
+  if (!pl) return;
+  cudaFree(pl->dU);
+  cudaFree(pl->dS);
+  cudaFree(pl->dYr);
+  cudaFree(pl->dCr);
+  delete pl;
+}
+
+void lmm_plan_load_k(gbm_lmm_plan* pl, const double* K, int64_t ldk) {
+  State& st = state();
+  const int64_t n = pl->n;
   if (pl->ldu != n) GBM_CUDA(cudaMemsetAsync(pl->dU, 0, sizeof(double) * pl->ldu * n, st.stream));
-  GBM_CUDA(cudaMemcpy2DAsync(pl->dU, pl->ldu * sizeof(double), K, n * sizeof(double), n * sizeof(double), n,
+  GBM_CUDA(cudaMemcpy2DAsync(pl->dU, pl->ldu * sizeof(double), K, ldk * sizeof(double), n * sizeof(double), n,
                              cudaMemcpyDefault, st.stream));
+}
+
+void lmm_plan_factor(gbm_lmm_plan* pl, const double* y, const double* C, int64_t k, int64_t ldc, double* eig_ms) {
+  State& st = state();
+  const int64_t n = pl->n;
+  const int Q0 = pl->Q0;
   // K = U S U' through cuSOLVER (lower triangle), timed separately
   if (!st.cusolver) {
     cusolverDnHandle_t h;
@@ -2114,8 +2109,25 @@ int gbm_lmm_plan_create(const double* K, int64_t n, const double* y, const doubl
   GBM_CUDA(cudaMemcpy(hC.data(), pl->dCr, sizeof(double) * n * Q0, cudaMemcpyDeviceToHost));
   pl->s_min = hS[0];
   pl->lam0 = lmm_null_lam0(Q0, hS.data(), hC.data(), n, hY.data(), n);
+}
+
+}  // namespace gbm
+
+extern "C" {
+
+int gbm_lmm_plan_create(const double* K, int64_t n, const double* y, const double* C, int64_t k, int64_t ldc,
+                        gbm_lmm_plan** plan_out, double* eig_ms, double* null_log_delta) {
+  GBM_API_BEGIN
+  require_ready();
+  if (!K || !y || !plan_out || n < 4) GBM_THROW(GBM_ERR_ARGUMENT, "gbm_lmm_plan_create: bad arguments");
+  if (k < 0 || k > 2 || (k > 0 && (!C || ldc < n)))
+    GBM_THROW(GBM_ERR_ARGUMENT, "gbm_lmm_plan_create: 0..2 covariates besides the intercept are supported");
+  if (n > 2147483647) GBM_THROW(GBM_ERR_ARGUMENT, "n too large for cuSOLVER");
+  reset_timing();
+  std::unique_ptr<gbm_lmm_plan, void (*)(gbm_lmm_plan*)> pl(lmm_plan_alloc(n, static_cast<int>(k) + 1), lmm_plan_destroy);
+  lmm_plan_load_k(pl.get(), K, n);
+  lmm_plan_factor(pl.get(), y, C, k, ldc, eig_ms);
   if (null_log_delta) *null_log_delta = pl->lam0;
-  guard.p = nullptr;
   *plan_out = pl.release();
   GBM_API_END
 }
@@ -2188,11 +2200,7 @@ int gbm_lmm_plan_free(gbm_lmm_plan* pl) {
   GBM_API_BEGIN
   if (pl) {
     if (state().ready) cudaStreamSynchronize(state().stream);
-    cudaFree(pl->dU);
-    cudaFree(pl->dS);
-    cudaFree(pl->dYr);
-    cudaFree(pl->dCr);
-    delete pl;
+    lmm_plan_destroy(pl);
   }
   GBM_API_END
 }

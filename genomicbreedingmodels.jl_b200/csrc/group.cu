@@ -18,6 +18,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <array>
 #include <chrono>
 #include <condition_variable>
 #include <functional>
@@ -770,6 +771,167 @@ std::pair<int64_t, double> sharded_colstats(gbm_sharded* m, const ColstatsOut& o
   }
 }
 
+void check_lmm_covariates(int64_t n, const double* C, int64_t k, int64_t ldc, const char* who) {
+  if (n < 4) GBM_THROW(GBM_ERR_ARGUMENT, std::string(who) + ": at least 4 entries are needed");
+  if (n > 2147483647) GBM_THROW(GBM_ERR_ARGUMENT, "n too large for cuSOLVER");
+  if (k < 0 || k > 2 || (k > 0 && (!C || ldc < n)))
+    GBM_THROW(GBM_ERR_ARGUMENT, std::string(who) + ": 0..2 covariates besides the intercept are supported");
+}
+
+}  // namespace
+
+struct gbm_sharded_lmm_plan {
+  gbm_group* grp = nullptr;
+  int64_t n = 0;
+  std::vector<gbm_lmm_plan*> local;  // per local GPU; the same bits on every GPU of the group
+  double eig_ms = 0.0;               // rank 0's syevd
+};
+
+namespace {
+
+void free_lmm_plan(gbm_sharded_lmm_plan* P) {
+  try {
+    P->grp->run([&](int g) {
+      if (!P->local[g]) return;
+      cudaStreamSynchronize(state().stream);
+      lmm_plan_destroy(P->local[g]);
+      P->local[g] = nullptr;
+    });
+  } catch (...) {
+  }
+}
+
+struct LmmFactorTimes {
+  double kprep_ms = 0, eig_ms = 0, broadcast_ms = 0;
+};
+
+// The eigendecomposition, once per group.  Every GPU allocates its plan, and rank 0 puts K into its U buffer
+// (load_k(plan, g), which may also transform it, *kprep_ms = its host time) and factors it, all in ONE G.phase: a
+// failure there (an allocation, syevd info != 0) is agreed on by every rank before the first broadcast, so nobody
+// waits in NCCL for a rank that has already returned.  Then U (ldu x n, padding included), S, U'y, U'[1, C] and the
+// scalars travel from rank 0 to everybody.
+gbm_sharded_lmm_plan* sharded_lmm_factor(gbm_group& G, int64_t n, const std::function<void(gbm_lmm_plan*, int)>& load_k,
+                                         const double* y, const double* C, int64_t k, int64_t ldc, LmmFactorTimes* t,
+                                         int64_t* launches) {
+  std::unique_ptr<gbm_sharded_lmm_plan> P(new gbm_sharded_lmm_plan);
+  P->grp = &G;
+  P->n = n;
+  P->local.assign(G.n_local, nullptr);
+  std::vector<std::unique_ptr<Dev<double>>> scal(G.n_local);  // lam0, s_min, eig_ms, kprep_ms
+  std::vector<std::array<double, 4>> h(G.n_local, std::array<double, 4>{0.0, 0.0, 0.0, 0.0});
+  try {
+    const double t0 = now_ms();
+    G.phase([&](int g) {
+      scal[g].reset(new Dev<double>(4));
+      P->local[g] = lmm_plan_alloc(n, static_cast<int>(k) + 1);
+      if (G.rank_of(g) != 0) return;
+      gbm_lmm_plan* pl = P->local[g];
+      const int64_t l0 = state().launches;
+      const double tk = now_ms();
+      load_k(pl, g);
+      GBM_CUDA(cudaStreamSynchronize(state().stream));
+      h[g][3] = now_ms() - tk;
+      lmm_plan_factor(pl, y, C, k, ldc, &h[g][2]);
+      h[g][0] = pl->lam0;
+      h[g][1] = pl->s_min;
+      if (launches) launches[g] += state().launches - l0;
+    });
+    const double t1 = now_ms();
+    G.run([&](int g) {
+      gbm_lmm_plan* pl = P->local[g];
+      cudaStream_t s = state().stream;
+      double* sc = scal[g]->p;
+      if (G.rank_of(g) == 0) GBM_CUDA(cudaMemcpyAsync(sc, h[g].data(), sizeof(double) * 4, cudaMemcpyHostToDevice, s));
+      if (G.world > 1) {
+        GBM_NCCL(nccl().GroupStart());
+        GBM_NCCL(nccl().Broadcast(pl->dU, pl->dU, static_cast<size_t>(pl->ldu) * n, ncclDouble, 0, G.comm[g], s));
+        GBM_NCCL(nccl().Broadcast(pl->dS, pl->dS, static_cast<size_t>(n), ncclDouble, 0, G.comm[g], s));
+        GBM_NCCL(nccl().Broadcast(pl->dYr, pl->dYr, static_cast<size_t>(n), ncclDouble, 0, G.comm[g], s));
+        GBM_NCCL(nccl().Broadcast(pl->dCr, pl->dCr, static_cast<size_t>(n) * pl->Q0, ncclDouble, 0, G.comm[g], s));
+        GBM_NCCL(nccl().Broadcast(sc, sc, 4, ncclDouble, 0, G.comm[g], s));
+        GBM_NCCL(nccl().GroupEnd());
+      }
+      GBM_CUDA(cudaMemcpyAsync(h[g].data(), sc, sizeof(double) * 4, cudaMemcpyDeviceToHost, s));
+      GBM_CUDA(cudaStreamSynchronize(s));
+      pl->lam0 = h[g][0];
+      pl->s_min = h[g][1];
+      scal[g].reset();
+    });
+    if (t) {
+      t->kprep_ms = h[0][3];
+      t->eig_ms = (t1 - t0) - h[0][3];
+      t->broadcast_ms = now_ms() - t1;
+    }
+  } catch (...) {
+    try {
+      G.run([&](int g) { scal[g].reset(); });
+    } catch (...) {
+    }
+    free_lmm_plan(P.get());
+    throw;
+  }
+  P->eig_ms = h[0][2];
+  return P.release();
+}
+
+struct LmmOut {
+  double *beta, *se, *stat, *nlp, *log_delta;
+};
+
+// the marker loop: every GPU runs gbm_lmm_plan_run on its own block (rotation in column blocks + delta search), then
+// the five per-marker outputs are gathered in locus order.  Fills the marker fields of *t.
+void sharded_lmm_run(gbm_sharded_lmm_plan* P, gbm_sharded* m, int flags, const LmmOut& o, gbm_reml_timing* t,
+                     int64_t* launches) {
+  gbm_group& G = *m->grp;
+  const int64_t p = m->p;
+  std::vector<std::vector<double>> dev_ms(G.n_local, std::vector<double>(2, 0.0));  // rotation, search
+  std::vector<BlockBufs> buf(G.n_local);
+  double* const want[5] = {o.beta, o.se, o.stat, o.nlp, o.log_delta};
+  const double t0 = now_ms();
+  try {
+    G.phase([&](int g) {
+      const int64_t pc = m->ncols[G.rank_of(g)];
+      BlockBufs& b = buf[g];
+      for (int i = 0; i < 5; ++i)
+        if (want[i]) b.d[i].reset(new Dev<double>(pc));
+      double tflops = 0.0, search_ms = 0.0;
+      ok(gbm_lmm_plan_run(P->local[g], m->local[g], flags, ptr_of(b.d[0]), ptr_of(b.d[1]), ptr_of(b.d[2]), ptr_of(b.d[3]),
+                          ptr_of(b.d[4]), &tflops, &search_ms));
+      dev_ms[g][0] = state().main_ms;  // the rotation GEMMs' events
+      dev_ms[g][1] = search_ms;
+      if (launches) launches[g] += state().launches;
+    });
+    const double t1 = now_ms();
+    G.run([&](int g) {
+      BlockBufs& b = buf[g];
+      for (int i = 0; i < 5; ++i) gather_rows(G, g, ptr_of(b.d[i]), m->ncols, m->col0, p, int64_t(1), want[i]);
+      GBM_CUDA(cudaStreamSynchronize(state().stream));
+      b.reset();
+    });
+    t->scan_ms = t1 - t0;
+    t->gather_ms = now_ms() - t1;
+  } catch (...) {
+    try {
+      G.run([&](int g) { buf[g].reset(); });
+    } catch (...) {
+    }
+    throw;
+  }
+  G.reduce_host(dev_ms, ncclMax);  // the slowest GPU
+  t->rotation_ms = dev_ms[0][0];
+  t->search_ms = dev_ms[0][1];
+  t->rotation_tflops = 2.0 * static_cast<double>(m->n) * static_cast<double>(m->n) * static_cast<double>(p) /
+                       (t->rotation_ms * 1e-3) / 1e12;
+  t->n_gpus = G.world;
+}
+
+void check_lmm_plan(const gbm_sharded_lmm_plan* P, const gbm_sharded* m) {
+  if (!P) GBM_THROW(GBM_ERR_ARGUMENT, "gbm_sharded_lmm_plan_run: null plan");
+  if (P->grp != m->grp) GBM_THROW(GBM_ERR_ARGUMENT, "gbm_sharded_lmm_plan_run: the plan belongs to another group");
+  if (P->n != m->n)
+    GBM_THROW(GBM_ERR_ARGUMENT, "gbm_sharded_lmm_plan_run: the matrix and the GRM have different numbers of entries");
+}
+
 }  // namespace
 
 #define GBM_GROUP_BEGIN try {
@@ -1142,6 +1304,121 @@ int gbm_sharded_gwas(gbm_sharded* m, const double* y, int model, int grm_type, i
   // marker loop with X = [1, PC1, g_j]  (gwas.jl:239-249 / :363-389)
   t.scan_kernel_ms = sharded_scan(m, y, 1, m->n, pc.data(), 1, m->n, model, flags & GBM_PVALUE_TWO_SIDED,
                                   ScanOut{beta, se, stat, neglog10p, mean, sd, keep}, &t.scan_ms, &t.gather_ms, launches.data());
+  t.total_ms = now_ms() - t0;
+  for (int64_t l : launches) t.launches += l;
+  if (timing) *timing = t;
+  GBM_GROUP_END
+}
+
+
+int gbm_sharded_lmm_plan_create(gbm_sharded* m, const double* K, const double* y, const double* C, int64_t k,
+                                int64_t ldc, gbm_sharded_lmm_plan** plan, double* eig_ms, double* null_log_delta) {
+  GBM_GROUP_BEGIN
+  check_sharded(m);
+  if (!K || !y || !plan) GBM_THROW(GBM_ERR_ARGUMENT, "gbm_sharded_lmm_plan_create: null pointer");
+  check_lmm_covariates(m->n, C, k, ldc, "gbm_sharded_lmm_plan_create");
+  std::lock_guard<std::mutex> lk(m->grp->mutex);
+  const int64_t n = m->n;
+  gbm_sharded_lmm_plan* P = sharded_lmm_factor(
+      *m->grp, n, [&](gbm_lmm_plan* pl, int) { lmm_plan_load_k(pl, K, n); }, y, C, k, ldc, nullptr, nullptr);
+  if (eig_ms) *eig_ms = P->eig_ms;
+  if (null_log_delta) *null_log_delta = P->local[0]->lam0;
+  *plan = P;
+  GBM_GROUP_END
+}
+
+int gbm_sharded_lmm_plan_run(gbm_sharded_lmm_plan* plan, gbm_sharded* m, int flags, double* beta, double* se,
+                             double* stat, double* neglog10p, double* log_delta, gbm_reml_timing* timing) {
+  GBM_GROUP_BEGIN
+  check_sharded(m);
+  check_lmm_plan(plan, m);
+  std::lock_guard<std::mutex> lk(m->grp->mutex);
+  std::vector<int64_t> launches(m->grp->n_local, 0);
+  gbm_reml_timing t;
+  memset(&t, 0, sizeof(t));
+  const double t0 = now_ms();
+  sharded_lmm_run(plan, m, flags, LmmOut{beta, se, stat, neglog10p, log_delta}, &t, launches.data());
+  t.total_ms = now_ms() - t0;
+  for (int64_t l : launches) t.launches += l;
+  if (timing) *timing = t;
+  GBM_GROUP_END
+}
+
+int gbm_sharded_lmm_plan_free(gbm_sharded_lmm_plan* plan) {
+  GBM_GROUP_BEGIN
+  if (!plan) return GBM_OK;
+  {
+    std::lock_guard<std::mutex> lk(plan->grp->mutex);
+    free_lmm_plan(plan);
+  }
+  delete plan;
+  GBM_GROUP_END
+}
+
+int gbm_sharded_gwasreml(gbm_sharded* m, const double* y, int grm_type, int flags, double* stat, double* beta,
+                         double* se, double* neglog10p, double* log_delta, int64_t* idx_cols, int64_t* n_keep,
+                         double* null_log_delta, gbm_reml_timing* timing) {
+  GBM_GROUP_BEGIN
+  check_sharded(m);
+  if (!y) GBM_THROW(GBM_ERR_ARGUMENT, "gbm_sharded_gwasreml: null trait vector");
+  if (grm_type != GBM_GRM_SIMPLE && grm_type != GBM_GRM_PLOIDY_AWARE)
+    GBM_THROW(GBM_ERR_ARGUMENT, "Unrecognised `GRM_type`. Please select from:\n\t‣ simple\n\t‣ ploidy-aware");
+  // one flags word for the scan only: the GRM is always centred (GBM_GRM_NO_CENTRE has the value of
+  // GBM_PVALUE_TWO_SIDED, so it cannot be passed here)
+  if (flags & ~(GBM_PVALUE_TWO_SIDED | GBM_LMM_REFERENCE_OBJECTIVE))
+    GBM_THROW(GBM_ERR_ARGUMENT, "gbm_sharded_gwasreml: flags may only hold GBM_PVALUE_TWO_SIDED and GBM_LMM_REFERENCE_OBJECTIVE");
+  check_lmm_covariates(m->n, nullptr, 0, m->n, "gbm_sharded_gwasreml");
+  gbm_group& G = *m->grp;
+  std::lock_guard<std::mutex> lk(G.mutex);
+  const int64_t n = m->n;
+  const bool ref = (flags & GBM_LMM_REFERENCE_OBJECTIVE) != 0;
+  std::vector<int64_t> launches(G.n_local, 0);
+  gbm_reml_timing t;
+  memset(&t, 0, sizeof(t));
+  const double t0 = now_ms();
+  // v = std(G, dims=1); idx_cols; minimum(G[G .!= 0])   (gwas.jl:112-113, :119)
+  const auto cs = sharded_colstats(m, ColstatsOut{nullptr, nullptr, nullptr, nullptr, idx_cols}, launches.data());
+  if (n_keep) *n_keep = cs.first;
+  int ploidy = 2;
+  if (grm_type == GBM_GRM_PLOIDY_AWARE) {
+    if (!(cs.second > 0.0)) GBM_THROW(GBM_ERR_RUNTIME, "cannot infer the ploidy: no non-zero allele frequency among the kept loci");
+    ploidy = static_cast<int>(nearbyint(1.0 / cs.second));  // Int(round(1 / minimum(G[G .!= 0.0])))
+  }
+  t.ploidy = ploidy;
+  t.colstats_ms = now_ms() - t0;
+  // GRM on all entries and loci (gwas.jl:117-126), resident on every GPU
+  const GrmTimes gt = sharded_grm(m, grm_type, ploidy, 0, launches.data());
+  t.grm_ms = gt.grm_ms;
+  t.allreduce_ms = gt.allreduce_ms;
+  t.grm_tflops = static_cast<double>(n) * static_cast<double>(n + 1) * static_cast<double>(m->p) /
+                 ((gt.grm_ms + gt.allreduce_ms) * 1e-3) / 1e12;
+  // rank 0: K into the plan's U buffer; for the reference objective K = (K .- mean(K, dims=1)) ./ std(K, dims=1)
+  // (gwas.jl:130, the kernels of gbm_kstd_pc1) and its symmetric part, the matrix a rotation can factor
+  auto load_k = [&](gbm_lmm_plan* pl, int g) {
+    lmm_plan_load_k(pl, m->dK[g], n);
+    if (!ref) return;
+    State& st = state();
+    const int stride = scan_record_stride(0, true);
+    Dev<double> rec(static_cast<size_t>(n) * stride), mean(n), sd(n);
+    launch_scan_sums(pl->dU, n, n, pl->ldu, nullptr, 0, 0, true, rec.p, st.sm_count, st.stream);
+    launch_colstats_finalize(rec.p, stride, n, n, mean.p, sd.p, nullptr, nullptr, st.stream);
+    launch_k_standardise(pl->dU, n, n, pl->ldu, mean.p, sd.p, st.stream);
+    launch_symmetrise(pl->dU, n, pl->ldu, st.stream);
+    st.launches += 4;
+  };
+  LmmFactorTimes ft;
+  std::unique_ptr<gbm_sharded_lmm_plan, int (*)(gbm_sharded_lmm_plan*)> P(
+      sharded_lmm_factor(G, n, load_k, y, nullptr, 0, n, &ft, launches.data()), [](gbm_sharded_lmm_plan* q) {
+        free_lmm_plan(q);
+        delete q;
+        return GBM_OK;
+      });
+  t.kprep_ms = ft.kprep_ms;
+  t.eig_ms = ft.eig_ms;
+  t.broadcast_ms = ft.broadcast_ms;
+  if (null_log_delta) *null_log_delta = P->local[0]->lam0;
+  // marker loop: rotation + delta search per GPU, gather in locus order (gwas.jl:586-607)
+  sharded_lmm_run(P.get(), m, flags, LmmOut{beta, se, stat, neglog10p, log_delta}, &t, launches.data());
   t.total_ms = now_ms() - t0;
   for (int64_t l : launches) t.launches += l;
   if (timing) *timing = t;

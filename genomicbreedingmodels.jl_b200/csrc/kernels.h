@@ -93,6 +93,8 @@ void launch_k_standardise(double* K, int64_t n, int64_t ncols, int64_t ld, const
 void launch_row_shift(double* Z, int64_t n, int64_t ncols, int64_t ld, const double* rowsum, double inv_cols,
                       cudaStream_t stream);
 void launch_row_centre(const double* Ks, double* Z, int64_t n, int64_t ld, cudaStream_t stream);
+// K <- (K + K') / 2 in place (n x n, pitch ld)
+void launch_symmetrise(double* K, int64_t n, int64_t ld, cudaStream_t stream);
 // gather rows/cols (1-based indices, nullable) from a device source into a padded device matrix
 void launch_gather(const double* src, int64_t lds, const int64_t* rows, int64_t n, const int64_t* cols, int64_t p,
                    double* dst, int64_t ldd, cudaStream_t stream);
@@ -198,4 +200,26 @@ int64_t transform_select(const double* beta_dev, int64_t len, int64_t n_new, dou
                          double* beta_host, bool* has_nan, int sm_count, cudaStream_t stream);
 void launch_gather_values(const double* src, const long long* idx1, int64_t count, double* dst, cudaStream_t stream);
 
+}  // namespace gbm
+
+// gbm_api.cu: the LMM plan (gbm_lmm_plan_*) in steps, shared by the single-GPU entry points and the group engine
+// (group.cu: rank 0 loads and factors K, the other GPUs receive U, S, U'y, U'[1, C], lam0 and s_min)
+struct gbm_lmm_plan {
+  int64_t n = 0, ldu = 0;
+  int Q0 = 1;
+  double* dU = nullptr;   // eigenvectors, n x n (ldu)
+  double* dS = nullptr;   // eigenvalues ascending
+  double* dYr = nullptr;  // U'y
+  double* dCr = nullptr;  // U'[1, C], n x Q0 (ld n)
+  double lam0 = 0.0;
+  double s_min = 0.0;     // smallest eigenvalue (negative for an indefinite K)
+};
+namespace gbm {
+// device buffers on the calling thread's GPU (ldu = n rounded up to 16); throws, leaving nothing allocated, on failure
+gbm_lmm_plan* lmm_plan_alloc(int64_t n, int Q0);
+void lmm_plan_destroy(gbm_lmm_plan* pl);
+// K (n x n, pitch ldk, host or device) into dU, padding rows zeroed
+void lmm_plan_load_k(gbm_lmm_plan* pl, const double* K, int64_t ldk);
+// dU holds K: K = U S U' (cuSOLVER syevd, eig_ms = its time), rotation of [1, C, y], null-model lam0 and s_min
+void lmm_plan_factor(gbm_lmm_plan* pl, const double* y, const double* C, int64_t k, int64_t ldc, double* eig_ms);
 }  // namespace gbm

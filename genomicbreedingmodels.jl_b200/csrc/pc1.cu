@@ -1,7 +1,7 @@
 // Element-wise kernels around the PC1 step of gwasols / gwaslmm:
 //   K = (K .- mean(K, dims=1)) ./ std(K, dims=1)                    /root/reference/src/gwas.jl:130
 //   MultivariateStats.fit(PCA, K; maxoutdim=1): centre the rows     /root/reference/src/gwas.jl:234, :357
-// and the gather behind `allele_frequencies[idx_entries[idx], idx_loci_alleles]`
+// the symmetric part of the standardised K (gwasreml's reference objective), and the gather behind `allele_frequencies[idx_entries[idx], idx_loci_alleles]`
 // (/root/reference/src/prediction.jl:129).  HBM-bound streaming kernels, 128-bit accesses
 // where the layout allows it.
 #include "common.cuh"
@@ -56,6 +56,34 @@ __global__ void __launch_bounds__(128)
 void launch_row_centre(const double* Ks, double* Z, int64_t n, int64_t ld, cudaStream_t stream) {
   if (n <= 0) return;
   row_centre_kernel<<<static_cast<unsigned>((n + 127) / 128), 128, 0, stream>>>(Ks, Z, n, ld);
+  GBM_CUDA(cudaGetLastError());
+}
+
+// K <- (K + K') / 2 in place: the symmetric part of the column-standardised GRM, the matrix the eigen-rotation of
+// gwasreml's reference objective factors.  One CTA per 32 x 32 tile pair (I, J), I >= J, both tiles through shared
+// memory before any store (the diagonal tile is its own partner); both entries get 0.5 * (a + b), the same bits in
+// either order.
+__global__ void __launch_bounds__(256) symmetrise_kernel(double* __restrict__ K, int64_t n, int64_t ld) {
+  __shared__ double a[32][33], b[32][33];
+  const int bi = blockIdx.x, bj = blockIdx.y;
+  if (bj > bi) return;
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;  // 32 x 8
+  const int64_t r0 = static_cast<int64_t>(bi) * 32, c0 = static_cast<int64_t>(bj) * 32;
+  for (int r = ty; r < 32; r += 8) {
+    a[r][tx] = (r0 + tx < n && c0 + r < n) ? K[(c0 + r) * ld + r0 + tx] : 0.0;  // tile (I, J): K[r0 + tx, c0 + r]
+    b[r][tx] = (c0 + tx < n && r0 + r < n) ? K[(r0 + r) * ld + c0 + tx] : 0.0;  // tile (J, I): K[c0 + tx, r0 + r]
+  }
+  __syncthreads();
+  for (int r = ty; r < 32; r += 8) {
+    if (r0 + tx < n && c0 + r < n) K[(c0 + r) * ld + r0 + tx] = 0.5 * (a[r][tx] + b[tx][r]);
+    if (c0 + tx < n && r0 + r < n) K[(r0 + r) * ld + c0 + tx] = 0.5 * (b[r][tx] + a[tx][r]);
+  }
+}
+
+void launch_symmetrise(double* K, int64_t n, int64_t ld, cudaStream_t stream) {
+  if (n <= 0) return;
+  const unsigned nb = static_cast<unsigned>((n + 31) / 32);
+  symmetrise_kernel<<<dim3(nb, nb), 256, 0, stream>>>(K, n, ld);
   GBM_CUDA(cudaGetLastError());
 }
 

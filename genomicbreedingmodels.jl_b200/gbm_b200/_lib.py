@@ -56,6 +56,17 @@ class GwasTiming(ctypes.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_}
 
 
+class RemlTiming(ctypes.Structure):
+    """gbm_reml_timing of include/gbm_b200.h"""
+    _fields_ = [("colstats_ms", c_double), ("grm_ms", c_double), ("allreduce_ms", c_double), ("kprep_ms", c_double),
+                ("eig_ms", c_double), ("broadcast_ms", c_double), ("scan_ms", c_double), ("gather_ms", c_double),
+                ("total_ms", c_double), ("rotation_ms", c_double), ("search_ms", c_double), ("rotation_tflops", c_double),
+                ("grm_tflops", c_double), ("launches", c_int64), ("ploidy", ctypes.c_int32), ("n_gpus", ctypes.c_int32)]
+
+    def asdict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
 class Timing(ctypes.Structure):
     _fields_ = [("h2d_ms", c_double), ("kernel_ms", c_double), ("main_ms", c_double), ("d2h_ms", c_double),
                 ("launches", c_int64), ("packed_blocks", c_int64), ("host_packed_blocks", c_int64), ("h2d_bytes", c_int64)]
@@ -128,6 +139,12 @@ SIGNATURES = {
                                  _P]),
     "gbm_sharded_gwas": (c_int, [c_void_p, _P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P, _P, _P, POINTER(c_int64), _P,
                                  POINTER(GwasTiming)]),
+    "gbm_sharded_lmm_plan_create": (c_int, [c_void_p, _P, _P, _P, c_int64, c_int64, POINTER(c_void_p), POINTER(c_double),
+                                            POINTER(c_double)]),
+    "gbm_sharded_lmm_plan_run": (c_int, [c_void_p, c_void_p, c_int, _P, _P, _P, _P, _P, POINTER(RemlTiming)]),
+    "gbm_sharded_lmm_plan_free": (c_int, [c_void_p]),
+    "gbm_sharded_gwasreml": (c_int, [c_void_p, _P, c_int, c_int, _P, _P, _P, _P, _P, _P, POINTER(c_int64), POINTER(c_double),
+                                     POINTER(RemlTiming)]),
     "gbm_neglog10_sf": (c_int, [_P, c_int64, c_int, c_double, _P]),
     "gbm_measure_copy_bandwidth": (c_int, [c_int64, c_int, POINTER(c_double)]),
 }

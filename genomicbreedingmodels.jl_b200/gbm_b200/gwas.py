@@ -353,6 +353,48 @@ def gwaslmm(*, genomes: Genomes, phenomes: Phenomes, idx_entries=None, idx_loci_
                  verbose)
 
 
+def _gwasreml_multigpu(group, genomes, phenomes, idx_trait, GRM_type, y, objective) -> Fit:
+    """gwasreml on a group of GPUs (GBM_NUM_GPUS > 1): markers sharded by column block, ONE collective call into the
+    library (gbm_sharded_upload + gbm_sharded_gwasreml); the same Fit as the single-GPU path, plus timing, n_gpus and
+    storage in extras."""
+    from .multigpu import ShardedMatrix
+
+    A = np.asarray(genomes.allele_frequencies, dtype=np.float64)
+    # the single-GPU path's y: standardised once for REML; for the reference objective gwasprep standardises it
+    # (gwas.jl:128) and gwasreml once more
+    ys = (y - y.mean()) / np.std(y, ddof=1)
+    if objective == "reference":
+        ys = (ys - ys.mean()) / np.std(ys, ddof=1)
+    sm = ShardedMatrix.upload(group, A, compact=True)
+    try:
+        res = sm.gwasreml(ys, grm_type=_lib.GRM_PLOIDY_AWARE if GRM_type == "ploidy-aware" else _lib.GRM_SIMPLE,
+                          objective=objective)
+        packed = sm.packed
+    finally:
+        sm.free()
+    idx_cols = res["idx_cols"]
+    sel = idx_cols - 1
+    if np.isnan(res["stat"][sel]).all() and np.isnan(A).any():
+        raise ErrorException("cannot convert a value of type Missing to Float64")
+    fit = Fit.new(A.shape[0], int(idx_cols.size))  # gwas.jl:133-140
+    fit.model = "GWAS_REML"  # :574
+    fit.trait = phenomes.traits[idx_trait - 1]
+    fit.b_hat_labels = [genomes.loci_alleles[j] for j in sel]
+    fit.entries = list(genomes.entries)
+    fit.populations = list(genomes.populations)
+    fit.metrics = {"": 0.0}
+    fit.b_hat = np.ascontiguousarray(res["stat"][sel])
+    tm = res["timing"]
+    fit.extras = {"beta": res["beta"][sel], "se": res["se"][sel], "neglog10p": res["neglog10p"][sel],
+                  "log_delta": res["log_delta"][sel], "null_log_delta": res["null_log_delta"], "idx_cols": idx_cols,
+                  "eig_ms": tm["eig_ms"], "gemm_tflops": tm["rotation_tflops"], "search_ms": tm["search_ms"],
+                  "ploidy": tm["ploidy"] if GRM_type == "ploidy-aware" else None, "objective": objective, "timing": tm,
+                  "n_gpus": group.world, "storage": "u8 dosage codes" if packed else "float64"}
+    if not fit.checkdims():  # :609-611
+        raise ErrorException("Error performing GWAS via REML using the " + GRM_type + " GRM.")
+    return fit
+
+
 def gwasreml(*, genomes: Genomes, phenomes: Phenomes, idx_entries=None, idx_loci_alleles=None, idx_trait: int = 1,
              GRM_type: str = "simple", verbose: bool = False, objective: str = "reml") -> Fit:
     """gwasreml (/root/reference/src/gwas.jl:549-613): per-marker LMM with the GRM as the
@@ -368,10 +410,24 @@ def gwasreml(*, genomes: Genomes, phenomes: Phenomes, idx_entries=None, idx_loci
       over [eps, 1]^2, no sigma^2 factor; :478, :588, :596-599) on the symmetric part of the column-standardised K
       that gwasprep hands to loglikreml (:130, :564-573) -- as close as a rotation-based engine can get; the
       non-symmetric part of that K and the L-BFGS path are what remains (oracle/lmm_oracle.py, DESIGN.md section 2).
-    PARITY UNPINNED either way."""
+    PARITY UNPINNED either way.
+
+    With ``GBM_NUM_GPUS`` > 1 and no entries or loci subset, the markers are sharded over that many GPUs: one
+    eigendecomposition on the first GPU, broadcast, every GPU rotates and searches its own markers."""
     if objective not in ("reml", "reference"):
         raise ArgumentError("objective must be \"reml\" or \"reference\"")
     ref = objective == "reference"
+    from .multigpu import default_group
+
+    group = default_group()  # GBM_NUM_GPUS > 1
+    if group is not None:
+        rows1, cols1, y = _validate_and_select(genomes, phenomes, idx_entries, idx_loci_alleles, idx_trait)
+        if GRM_type not in GRM_TYPES:
+            raise ArgumentError("Unrecognised `GRM_type`. Please select from:\n\t‣ " + "\n\t‣ ".join(GRM_TYPES))
+        if np.var(y, ddof=1) < _EPS:
+            raise ArgumentError("No variance in the trait: " + phenomes.traits[idx_trait - 1] + ".")
+        if rows1 is None and cols1 is None and np.shape(genomes.allele_frequencies)[1] >= group.world:
+            return _gwasreml_multigpu(group, genomes, phenomes, idx_trait, GRM_type, y, objective)
     pr = _prepare(genomes, phenomes, idx_entries, idx_loci_alleles, idx_trait, GRM_type, ref, need_kstd=ref,
                   need_pc1=False)  # gwas.jl:564-573 (reml: K stays symmetric, standardise=False)
     try:

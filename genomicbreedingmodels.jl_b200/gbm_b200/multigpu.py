@@ -216,12 +216,81 @@ class ShardedMatrix:
         out.update(keep=out["_keep"].view(bool), idx_cols=out["_idx"][: nk.value], timing=tm.asdict())
         return out
 
+    def lmm_plan(self, K, y, C=None) -> "ShardedLmmPlan":
+        """The GRM-covariance LMM of ``LmmPlan`` over the shards (``gbm_sharded_lmm_plan_create``): K is factored once,
+        on rank 0, and U is broadcast to every GPU.  Every process passes the same K, y and C."""
+        return ShardedLmmPlan(self, K, y, C)
+
+    def gwasreml(self, y, grm_type: int = _lib.GRM_SIMPLE, objective: str = "reml", two_sided: bool = False):
+        """Whole gwasreml after extractxyetc in ONE collective call (``gbm_sharded_gwasreml``): filter + ploidy probe,
+        GRM + all-reduce, for ``objective="reference"`` the symmetric part of the column-standardised K, the
+        eigendecomposition on rank 0 and its broadcast, rotation + delta search per GPU, gather.  ``y`` is used as
+        given."""
+        if objective not in ("reml", "reference"):
+            raise _lib.ArgumentError("objective must be \"reml\" or \"reference\"")
+        y = np.ascontiguousarray(y, dtype=np.float64)
+        if y.shape != (self.n,):
+            raise _lib.ArgumentError("phenotype length does not match the number of entries")
+        flags = (_lib.LMM_REFERENCE_OBJECTIVE if objective == "reference" else 0) | (
+            _lib.PVALUE_TWO_SIDED if two_sided else 0)
+        p = self.p
+        out = {k: np.empty(p) for k in ("stat", "beta", "se", "neglog10p", "log_delta")}
+        idx = np.empty(p, dtype=np.int64)
+        nk, lam0 = c_int64(), c_double()
+        tm = _lib.RemlTiming()
+        check(_lib.load().gbm_sharded_gwasreml(self._h, ptr(y), grm_type, flags, ptr(out["stat"]), ptr(out["beta"]),
+                                               ptr(out["se"]), ptr(out["neglog10p"]), ptr(out["log_delta"]), ptr(idx),
+                                               byref(nk), byref(lam0), byref(tm)))
+        out.update(idx_cols=idx[: nk.value].copy(), null_log_delta=lam0.value, timing=tm.asdict())
+        return out
+
+
+class ShardedLmmPlan:
+    """``gbm_sharded_lmm_plan``: the same interface as ``LmmPlan``, for a ``ShardedMatrix``."""
+
+    def __init__(self, sm: ShardedMatrix, K, y, C=None):
+        n = sm.n
+        y = np.ascontiguousarray(y, dtype=np.float64)
+        if y.shape != (n,):
+            raise _lib.ArgumentError("phenotype length does not match the number of entries")
+        K = _f64(K)
+        if K.shape != (n, n):
+            raise _lib.ArgumentError("GRM must be n x n")
+        Cm = None if C is None else _f64(np.asarray(C, dtype=np.float64).reshape(n, -1))
+        h = c_void_p()
+        eig, lam0 = c_double(), c_double()
+        check(_lib.load().gbm_sharded_lmm_plan_create(sm._h, ptr(K), ptr(y), ptr(Cm), 0 if Cm is None else Cm.shape[1], n,
+                                                      byref(h), byref(eig), byref(lam0)))
+        self._h, self.n, self._sm = h, n, sm
+        self.eig_ms, self.null_log_delta = eig.value, lam0.value
+
+    def run(self, flags: int = 0):
+        p = self._sm.p
+        out = {k: np.empty(p) for k in ("beta", "se", "stat", "neglog10p", "log_delta")}
+        tm = _lib.RemlTiming()
+        check(_lib.load().gbm_sharded_lmm_plan_run(self._h, self._sm._h, flags, ptr(out["beta"]), ptr(out["se"]),
+                                                   ptr(out["stat"]), ptr(out["neglog10p"]), ptr(out["log_delta"]),
+                                                   byref(tm)))
+        out["timing"] = tm.asdict()
+        return out
+
+    def free(self):
+        if self._h is not None:
+            check(_lib.load().gbm_sharded_lmm_plan_free(self._h))
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass
+
 
 _default_group = None
 
 
 def default_group():
-    """The group the host mirror's gwasols / gwaslmm use: ``GBM_NUM_GPUS`` GPUs of this process (None when the
+    """The group the host mirror's gwasols / gwaslmm / gwasreml use: ``GBM_NUM_GPUS`` GPUs of this process (None when the
     variable is unset or 1)."""
     global _default_group
     n = int(os.environ.get("GBM_NUM_GPUS", "1") or "1")

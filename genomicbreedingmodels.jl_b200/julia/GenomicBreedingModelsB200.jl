@@ -327,11 +327,62 @@ gwaslmm(; genomes::Genomes, phenomes::Phenomes, idx_entries::Union{Nothing,Vecto
 # What a rotation-based engine cannot reproduce (the non-symmetric part of that K, the L-BFGS path) is quantified in
 # oracle/lmm_oracle.py and DESIGN.md section 2.
 const GBM_LMM_REFERENCE_OBJECTIVE = Cint(8)
+
+struct RemlTiming   # gbm_reml_timing of include/gbm_b200.h
+    colstats_ms::Float64; grm_ms::Float64; allreduce_ms::Float64; kprep_ms::Float64; eig_ms::Float64
+    broadcast_ms::Float64; scan_ms::Float64; gather_ms::Float64; total_ms::Float64; rotation_ms::Float64
+    search_ms::Float64; rotation_tflops::Float64; grm_tflops::Float64; launches::Int64; ploidy::Int32; n_gpus::Int32
+end
+
+# GBM_NUM_GPUS > 1: the markers sharded over the group, K factored once on the first GPU and U broadcast
+# (gbm_sharded_gwasreml); the same Fit as the single-GPU path below.
+function gwasreml_multigpu(genomes, phenomes, idx_trait, GRM_type, y, ref::Bool)::Fit
+    A = Matrix{Float64}(genomes.allele_frequencies)       # throws on `missing`, as src/prediction.jl:129 does
+    n, p = size(A)
+    sm = Ref{Ptr{Cvoid}}(C_NULL); packed = Ref{Cint}(0)
+    check(ccall((:gbm_sharded_upload, LIBGBM), Cint,
+                (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Int64, Cint, Ref{Ptr{Cvoid}}, Ref{Cint}), group(), A, n, p, n, 1, sm, packed))
+    ys = (y .- mean(y)) ./ std(y)                         # src/gwas.jl:128; gwasreml standardises once more below
+    ref && (ys = (ys .- mean(ys)) ./ std(ys))             # (the reference objective's y went through gwasprep first)
+    stat = Vector{Float64}(undef, p); idx = Vector{Int64}(undef, p); nk = Ref{Int64}(0); lam0 = Ref{Float64}(0.0)
+    tm = Ref{RemlTiming}()
+    rc = ccall((:gbm_sharded_gwasreml, LIBGBM), Cint,
+               (Ptr{Cvoid}, Ptr{Float64}, Cint, Cint, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+                Ptr{Int64}, Ref{Int64}, Ref{Float64}, Ref{RemlTiming}),
+               sm[], ys, GRM_type == "ploidy-aware" ? GBM_GRM_PLOIDY_AWARE : GBM_GRM_SIMPLE,
+               ref ? GBM_LMM_REFERENCE_OBJECTIVE : Cint(0), stat, C_NULL, C_NULL, C_NULL, C_NULL, idx, nk, lam0, tm)
+    ccall((:gbm_sharded_free, LIBGBM), Cint, (Ptr{Cvoid},), sm[])
+    check(rc)
+    idx_cols = idx[1:nk[]]
+    fit = Fit(n = n, l = length(idx_cols))                # src/gwas.jl:133-140
+    fit.model = "GWAS_REML"                               # src/gwas.jl:574
+    fit.trait = phenomes.traits[idx_trait]
+    fit.b_hat_labels = genomes.loci_alleles[idx_cols]
+    fit.entries = genomes.entries
+    fit.populations = genomes.populations
+    fit.metrics = Dict("" => 0.0)
+    fit.b_hat = stat[idx_cols]                            # src/gwas.jl:599
+    if !checkdims(fit)                                    # src/gwas.jl:609-611
+        throw(ErrorException("Error performing GWAS via REML using the " * GRM_type * " GRM."))
+    end
+    fit
+end
+
 function gwasreml(; genomes::Genomes, phenomes::Phenomes, idx_entries::Union{Nothing,Vector{Int64}} = nothing,
     idx_loci_alleles::Union{Nothing,Vector{Int64}} = nothing, idx_trait::Int64 = 1, GRM_type::String = "simple",
     verbose::Bool = false, objective::String = "reml")::Fit
     objective in ("reml", "reference") || throw(ArgumentError("objective must be \"reml\" or \"reference\""))
     ref = objective == "reference"
+    if numgpus() > 1
+        rows, cols, y = selectrows(genomes, phenomes, idx_entries, idx_loci_alleles, idx_trait)
+        if sum(["simple", "ploidy-aware"] .== GRM_type) == 0
+            throw(ArgumentError("Unrecognised `GRM_type`. Please select from:\n\t‣ simple\n\t‣ ploidy-aware"))
+        end
+        var(y) < eps(Float64) && throw(ArgumentError("No variance in the trait: " * phenomes.traits[idx_trait] * "."))
+        if isnothing(rows) && isnothing(cols) && size(genomes.allele_frequencies, 2) >= numgpus()
+            return gwasreml_multigpu(genomes, phenomes, idx_trait, GRM_type, y, ref)
+        end
+    end
     pr = prepare(genomes, phenomes, idx_entries, idx_loci_alleles, idx_trait, GRM_type, ref; need_kstd = ref, need_pc1 = false)
     if length(pr.entries) != size(pr.K, 1)
         free!(pr.dm)

@@ -363,6 +363,44 @@ int gbm_sharded_gwas(gbm_sharded* m, const double* y, int model, int grm_type, i
                      double* se, double* neglog10p, double* mean, double* sd, uint8_t* keep, int64_t* idx_cols,
                      int64_t* n_keep, double* pc1, gbm_gwas_timing* timing);
 
+/* The GRM-covariance LMM (gbm_lmm_plan_*, the model of gwasreml) over the shards.  K is factored ONCE: rank 0 runs
+ * the syevd of gbm_lmm_plan_create, rotates [1, C, y] and fits the null model, then broadcasts U, S, U'y, U'[1, C],
+ * the null log(delta) and the smallest eigenvalue to every GPU -- U is the same bits everywhere.  Every GPU then
+ * rotates and searches its own column block exactly as gbm_lmm_plan_run does (no exchange); results are gathered in
+ * locus order, so per-marker outputs equal the single-GPU engine's for the same K. */
+typedef struct gbm_sharded_lmm_plan gbm_sharded_lmm_plan;
+/* host wall clock (ms) of each step of one collective call; steps a call does not run stay 0.  kprep: K into rank 0's
+ * factor buffer (standardised and symmetrised for the reference objective); eig: the plans' allocation, rank 0's
+ * syevd, rotation of [1, C, y] and null model; broadcast: U, S and the rest to every GPU; scan: rotation + search on
+ * every GPU; gather: the outputs in locus order */
+typedef struct gbm_reml_timing {
+  double colstats_ms, grm_ms, allreduce_ms, kprep_ms, eig_ms, broadcast_ms, scan_ms, gather_ms, total_ms;
+  double rotation_ms;     /* slowest GPU's rotation GEMMs U'A (CUDA events) */
+  double search_ms;       /* slowest GPU's per-marker delta search (CUDA events) */
+  double rotation_tflops; /* 2 n^2 p / rotation_ms: aggregate of the group */
+  double grm_tflops;      /* n(n+1)p / (grm_ms + allreduce_ms): aggregate of the group */
+  int64_t launches;       /* kernels launched by this process */
+  int32_t ploidy, n_gpus; /* ploidy the GRM used; GPUs of the group (all ranks) */
+} gbm_reml_timing;
+/* collective.  K: host n x n, the same on every process (only rank 0 reads it, lower triangle); y: n; C: n x k
+ * (ldc), k = 0..2 covariates besides the intercept -- as gbm_lmm_plan_create.  eig_ms: rank 0's syevd. */
+int gbm_sharded_lmm_plan_create(gbm_sharded* m, const double* K, const double* y, const double* C, int64_t k,
+                                int64_t ldc, gbm_sharded_lmm_plan** plan, double* eig_ms, double* null_log_delta);
+/* collective.  Outputs host, length p, locus order, on every process, nullable; flags as gbm_lmm_plan_run
+ * (GBM_PVALUE_TWO_SIDED, GBM_LMM_REFERENCE_OBJECTIVE).  timing (nullable): the marker steps only. */
+int gbm_sharded_lmm_plan_run(gbm_sharded_lmm_plan* plan, gbm_sharded* m, int flags, double* beta, double* se,
+                             double* stat, double* neglog10p, double* log_delta, gbm_reml_timing* timing);
+int gbm_sharded_lmm_plan_free(gbm_sharded_lmm_plan* plan);
+/* The whole of gwasreml (gwas.jl:549-613) after extractxyetc in one collective call: filter + ploidy probe, GRM
+ * (+ all-reduce; centred, never GBM_GRM_NO_CENTRE), with GBM_LMM_REFERENCE_OBJECTIVE the column standardisation of K
+ * (gwas.jl:130) and its symmetric part (K + K') / 2 on the device, then the plan above.  y: n, used as given.  flags:
+ * GBM_PVALUE_TWO_SIDED and GBM_LMM_REFERENCE_OBJECTIVE only, any other bit is an argument error.  Outputs (host,
+ * nullable): stat / beta / se / neglog10p / log_delta of length p in locus order (NaN for filtered markers),
+ * idx_cols (room for p), the null model's log(delta). */
+int gbm_sharded_gwasreml(gbm_sharded* m, const double* y, int grm_type, int flags, double* stat, double* beta,
+                         double* se, double* neglog10p, double* log_delta, int64_t* idx_cols, int64_t* n_keep,
+                         double* null_log_delta, gbm_reml_timing* timing);
+
 /* -log10 upper-tail probabilities on the device (log-space; finite where 1 - cdf saturates) */
 int gbm_neglog10_sf(const double* stat, int64_t len, int dist /*0: TDist(df), 1: Normal*/, double df, double* out);
 
