@@ -13,7 +13,7 @@ pytestmark = pytest.mark.gpu
     (128, 1000, synth.KIND_TETRAPLOID),  # one tile, ragged marker tail
     (300, 4097, synth.KIND_DIPLOID),     # 6 tiles, ragged rows and markers
     (129, 40000, synth.KIND_TETRAPLOID), # two accumulation slices (32768 + 7232 markers)
-    (1000, 70000, synth.KIND_DIPLOID),   # 36 tiles x 3 slices: more work items than SMs
+    (1000, 70000, synth.KIND_DIPLOID),   # 20 tiles x 3 slices = 60 work items (test_gpu_waves.py: past the first wave)
 ])
 def test_int8_grm_matches_oracle(gbm, n, p, kind):
     A = synth.block(31, n, 0, p, kind)
